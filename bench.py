@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the B200-native SG-SLAM tracking hot path (driver contract in the task statement).
 
-  python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--config s2|720p|hamming]
+  python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--config s2|720p|hamming] [--dump-outputs DIR]
 
 config s2 (default; BASELINE.json configs[1], the configuration `metric` is quoted on): one "step" = one pass of the hot path over a batch of
 synthetic 640x480 frames per GPU,
@@ -429,7 +429,12 @@ def main():
     ap.add_argument('--no-pipeline', action='store_true', help='e2e: skip the steps-in-flight mode')
     ap.add_argument('--pipeline-handles', type=int, default=3, help='e2e: full-size handles taking whole steps in turn')
     ap.add_argument('--no-detector', action='store_true', help='tracker-only step with ground-truth boxes (the round-1 definition of the step)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed to DIR/<name>.npy (see dump_step_outputs)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or args.config == 'hamming'):
+        ap.error('--dump-outputs writes the outputs of the GPU step: --impl ours with --config s2 or 720p')
     claim_stdout()
     cfg = CONFIGS.get(args.config)
     if args.impl == 'reference':
@@ -567,6 +572,8 @@ def main():
     sampler = ClockSampler(local); sampler.start(); time.sleep(0.3)
     total_ms = timed_steps(use_det, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_step_outputs(args.dump_outputs, L, B, trk, NB, cap, use_det)
     value = world * NB * args.steps / (total_ms * 1e-3)
     # ---- the tracker-only step (ground-truth boxes as inputs: the round-1 definition), with per-stage device times -------
     B.check(L.sgs_extractor_set_profiling(exh, 1))
@@ -893,6 +900,44 @@ def main():
         emit(line)
     if dist is not None:
         dist.destroy_process_group()
+
+
+DUMP_FRAMES = 128
+
+
+def dump_step_outputs(out_dir, L, B, trk, nb, cap, with_det):
+    """Writes what the last timed step left in the tracker -- what a caller of sgs_tracker_results_device (and sgs_tracker_boxes_device when the
+    detector is in the step) receives -- as float32 / float64 .npy files under out_dir, at most 64 MB in all.  Per-frame arrays cover
+    every frame; per-keypoint arrays cover a fixed sample of DUMP_FRAMES frames (seed 0, listed in sample_frames.npy), with the rows past a frame's
+    count zeroed (they are scratch, not results).  The inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    import torch
+    torch.cuda.synchronize()
+    p = [C.c_void_p() for _ in range(7)]
+    B.check(L.sgs_tracker_results_device(trk.h, *[C.byref(x) for x in p]))
+    counts = B.memcpy_d2h(np.zeros(nb, np.int32), p[3].value)
+    sample = np.sort(np.random.default_rng(0).choice(nb, min(nb, DUMP_FRAMES), replace=False))
+    valid = np.arange(cap)[None, :] < counts[sample, None]
+    kps = B.memcpy_d2h(np.zeros((nb, cap), B.KP_DTYPE), p[0].value)[sample]
+    out = {'counts': counts.astype(np.float64), 'nmatches': B.memcpy_d2h(np.zeros(nb, np.int32), p[5].value).astype(np.float64),
+           'sample_frames': sample.astype(np.float64),
+           'desc': np.where(valid[..., None], B.memcpy_d2h(np.zeros((nb, cap, 32), np.uint8), p[1].value)[sample], 0).astype(np.float32),
+           'u_right': np.where(valid, B.memcpy_d2h(np.zeros((nb, cap), np.float32), p[2].value)[sample], 0).astype(np.float32),
+           'cur_mp': np.where(valid, B.memcpy_d2h(np.zeros((nb, cap), np.int32), p[4].value)[sample], 0).astype(np.float64)}
+    for f in B.KP_DTYPE.names:
+        out['kp_' + f] = np.where(valid, kps[f], 0).astype(np.float32 if kps[f].dtype == np.float32 else np.float64)
+    if with_det:
+        pb, pn, ph = C.c_void_p(), C.c_void_p(), C.c_void_p()
+        B.check(L.sgs_tracker_boxes_device(trk.h, C.byref(pb), C.byref(pn), C.byref(ph)))
+        nboxes = B.memcpy_d2h(np.zeros(nb, np.int32), pn.value)
+        boxes = B.memcpy_d2h(np.zeros((nb, trk.max_boxes, 4), np.float32), pb.value)
+        boxes[np.arange(trk.max_boxes)[None, :] >= nboxes[:, None]] = 0
+        out['boxes'], out['nboxes'] = boxes, nboxes.astype(np.float64)
+        out['have_dyn'] = B.memcpy_d2h(np.zeros(nb, np.uint8), ph.value).astype(np.float64)
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+    log('[bench] outputs of the last timed step written to %s (%.1f MB)' % (out_dir, sum(a.nbytes for a in out.values()) / 1e6))
 
 
 def detector_gemm_table(det, kernel_ms, ncalls, nframes):

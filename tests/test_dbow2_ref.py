@@ -2,7 +2,7 @@
 tree against a cv::Mat stand-in, recipe in oracle/Makefile): a vocabulary trained by the real `create`, written by the real `saveToTextFile` /
 `saveToBinaryFile`, read back by the product's readers; the oracle's transform / BowVector / FeatureVector / DescriptorDistance compared with the
 real `transform(features, BowVector&, FeatureVector&, levelsup)`, `FORB::distance` -- everything exact (ids, node order, doubles bit for bit).
-No device needed.  Skipped only when the library was never built (the reference tree is absent AND no prebuilt copy travelled)."""
+No device needed.  The library's answers are replayed from tests/golden/ref (tests/refgolden.py)."""
 import ctypes as C
 import os
 
@@ -10,6 +10,7 @@ import numpy as np
 import pytest
 
 import oracle as O
+import refgolden as RG
 from pysgs import binding as B
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -17,14 +18,12 @@ REF_SO = os.path.join(ROOT, 'oracle', '_ref', 'libdbow2_ref.so')
 
 
 def _p(a):
-    return a.ctypes.data_as(C.c_void_p)
+    return RG.ptr(a)
 
 
 @pytest.fixture(scope='module')
 def ref():
-    if not os.path.exists(REF_SO):
-        pytest.skip('oracle/_ref/libdbow2_ref.so not built (needs /root/reference at build time)')
-    L = C.CDLL(REF_SO)
+    L = RG.load(REF_SO, __name__)
     for f in ('dbow2_ref_create', 'dbow2_ref_load_text', 'dbow2_ref_load_binary'):
         getattr(L, f).restype = C.c_void_p
     L.dbow2_ref_score.restype = C.c_double

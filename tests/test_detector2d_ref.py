@@ -12,18 +12,18 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, 'oracle'))
 import detector_oracle as DO  # noqa: E402
+import refgolden as RG  # noqa: E402
 
 LIB = os.path.join(ROOT, 'oracle', '_ref', 'libdetector2d_ref.so')
-pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason='oracle/_ref/libdetector2d_ref.so not built (reference tree absent)')
 
 
 def ref_post(rows, w, h, det_thr, dyn_thr):
-    L = C.CDLL(LIB)
+    L = RG.load(LIB, __name__)
     rows = np.ascontiguousarray(rows, np.float32).reshape(-1, 6)
     cap = max(1, len(rows))
     tv = np.zeros((cap, 6), np.float32); ob = np.zeros((cap, 6), np.float32); dm = np.zeros((cap, 4), np.float32); dr = np.zeros((cap, 4), np.float32)
     n = [C.c_int() for _ in range(6)]
-    p = lambda a: a.ctypes.data_as(C.c_void_p)
+    p = RG.ptr
     L.ref_detector2d_postprocess(len(rows), p(rows), w, h, C.c_float(det_thr), C.c_float(dyn_thr), cap, p(tv), C.byref(n[0]), p(ob), C.byref(n[1]), p(dm), C.byref(n[2]),
                                  p(dr), C.byref(n[3]), C.byref(n[4]), C.byref(n[5]))
     return tv[:n[0].value], ob[:n[1].value], dm[:n[2].value], dr[:n[3].value], bool(n[4].value), bool(n[5].value)

@@ -18,13 +18,12 @@ import ctypes as C
 import os
 
 import numpy as np
-import pytest
 
 import oracle as O
+import refgolden as RG
 from pysgs import synth
 
 LIB = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'oracle', '_ref', 'libframe_ref.so')
-pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason='oracle/_ref/libframe_ref.so not built (reference tree absent)')
 
 W, H, NF = 640, 480, 1000
 CAM = synth.TUM3
@@ -41,7 +40,7 @@ class Det:
 
 
 def _lib():
-    L = C.CDLL(LIB)
+    L = RG.load(LIB, __name__)
     L.ref_frame_push.restype = C.c_int; L.ref_frame_features_in_area.restype = C.c_int; L.ref_frame_is_in_frustum.restype = C.c_int
     return L
 
@@ -51,18 +50,18 @@ def run_reference(frames, depth, dets, dist5=NODIST, cam=CAM):
     L.ref_set_monotone_allocator(1)          # quadtree ties by creation order (quirk Q1, tests/test_orbextractor_ref.py)
     L.ref_frame_reset(NF, C.c_float(1.2), 8, 20, 7)
     K4 = np.array([cam['fx'], cam['fy'], cam['cx'], cam['cy']], np.float32)
-    d = np.ascontiguousarray(depth, np.float32); v = C.c_void_p
+    d = np.ascontiguousarray(depth, np.float32)
     out = []
     cap = 4 * NF
     for img, det in zip(frames, dets):
         img = np.ascontiguousarray(img, np.uint8)
         k = np.zeros(cap, O.KP_DTYPE); ku = np.zeros(cap, O.KP_DTYPE); ds = np.zeros((cap, 32), np.uint8)
         ur = np.zeros(cap, np.float32); dz = np.zeros(cap, np.float32); flags = np.zeros(8, np.int32); bounds = np.zeros(6, np.float32)
-        n = L.ref_frame_push(img.ctypes.data_as(v), W, H, d.ctypes.data_as(v), K4.ctypes.data_as(v), np.ascontiguousarray(dist5, np.float32).ctypes.data_as(v),
+        n = L.ref_frame_push(RG.ptr(img), W, H, RG.ptr(d), RG.ptr(K4), RG.ptr(np.ascontiguousarray(dist5, np.float32)),
                              C.c_float(cam['bf']), C.c_float(40.0), det.nobjects, int(det.have_rm), int(det.have_map),
-                             det.rm_boxes.ctypes.data_as(v), len(det.rm_boxes), det.map_boxes.ctypes.data_as(v), len(det.map_boxes),
-                             k.ctypes.data_as(v), ku.ctypes.data_as(v), ds.ctypes.data_as(v), ur.ctypes.data_as(v), dz.ctypes.data_as(v), cap,
-                             flags.ctypes.data_as(v), bounds.ctypes.data_as(v))
+                             RG.ptr(det.rm_boxes), len(det.rm_boxes), RG.ptr(det.map_boxes), len(det.map_boxes),
+                             RG.ptr(k), RG.ptr(ku), RG.ptr(ds), RG.ptr(ur), RG.ptr(dz), cap,
+                             RG.ptr(flags), RG.ptr(bounds))
         assert 0 <= n <= cap
         out.append(dict(n=n, keys=k[:n].copy(), keys_un=ku[:n].copy(), desc=ds[:flags[4]].copy(), u_right=ur[:n].copy(), depth=dz[:n].copy(),
                         have_rm=int(flags[0]), have_map=int(flags[1]), pre_have=int(flags[2]), pre_nboxes=int(flags[3]), bounds=bounds.copy()))
@@ -214,7 +213,7 @@ def test_grid_queries_and_frustum_of_the_reference_frame():
         x, y = rng.uniform(-30, W + 30), rng.uniform(-30, H + 30)
         r = float(rng.choice([4.0, 7.5, 15.0, 40.0, 90.0]))
         lo, hi = (-1, -1) if q % 3 == 0 else (int(rng.randint(0, 4)), int(rng.randint(3, 8)))
-        n = L.ref_frame_features_in_area(C.c_float(x), C.c_float(y), C.c_float(r), lo, hi, buf.ctypes.data_as(C.c_void_p), len(buf))
+        n = L.ref_frame_features_in_area(C.c_float(x), C.c_float(y), C.c_float(r), lo, hi, RG.ptr(buf), len(buf))
         got = O.features_in_area(fa, np.float32(x), np.float32(y), np.float32(r), lo, hi)
         assert n == len(got) and np.array_equal(buf[:n], got), q
         total += n
@@ -230,8 +229,8 @@ def test_grid_queries_and_frustum_of_the_reference_frame():
     dist = np.linalg.norm(xyz - Ow, axis=1).astype(np.float32)
     mx = (dist * rng.uniform(0.6, 3.0, npt)).astype(np.float32); mn = (mx / np.float32(1.2 ** 7)).astype(np.float32)
     out = np.zeros((npt, 6), np.float32)
-    cnt = L.ref_frame_is_in_frustum(T.ctypes.data_as(C.c_void_p), C.c_float(0.5), npt, xyz.ctypes.data_as(C.c_void_p), nrm.ctypes.data_as(C.c_void_p),
-                                    mn.ctypes.data_as(C.c_void_p), mx.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p))
+    cnt = L.ref_frame_is_in_frustum(RG.ptr(T), C.c_float(0.5), npt, RG.ptr(xyz), RG.ptr(nrm),
+                                    RG.ptr(mn), RG.ptr(mx), RG.ptr(out))
     cam = (CAM['fx'], CAM['fy'], CAM['cx'], CAM['cy'], CAM['bf'], 0.0, 0.0, float(W), float(H))
     want = O.is_in_frustum(T, cam, 8, float(O.logf(np.float32(1.2))), xyz, nrm, mn, mx, 0.5)
     assert cnt == int(want['inview'].sum()) and 100 < cnt < npt - 100

@@ -7,20 +7,18 @@ import ctypes as C
 import os
 
 import numpy as np
-import pytest
 
 import oracle as O
+import refgolden as RG
 
 LIB = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'oracle', '_ref', 'libmappoint_ref.so')
-pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason='oracle/_ref/libmappoint_ref.so not built (reference tree absent)')
-v = C.c_void_p
 
 
 def ref_distinctive(desc, bad=None):
-    L = C.CDLL(LIB); L.ref_mp_distinctive.restype = C.c_int
+    L = RG.load(LIB, __name__); L.ref_mp_distinctive.restype = C.c_int
     d = np.ascontiguousarray(desc, np.uint8); out = np.zeros(32, np.uint8)
     b = None if bad is None else np.ascontiguousarray(bad, np.uint8)
-    ok = L.ref_mp_distinctive(d.ctypes.data_as(v), b.ctypes.data_as(v) if b is not None else None, len(d), out.ctypes.data_as(v))
+    ok = L.ref_mp_distinctive(RG.ptr(d), RG.ptr(b) if b is not None else None, len(d), RG.ptr(out))
     return out if ok else None
 
 
@@ -51,7 +49,7 @@ def test_distinctive_descriptor_incl_ties_and_bad_key_frames():
 
 
 def test_predict_scale_and_invariance_getters():
-    L = C.CDLL(LIB)
+    L = RG.load(LIB, __name__)
     rng = np.random.RandomState(5)
     nlevels = 8
     log_sf = float(O.logf(np.float32(1.2)))
@@ -67,7 +65,7 @@ def test_predict_scale_and_invariance_getters():
                             (mx / rng.uniform(0.84, 6.0, 4000)).astype(np.float32)]).astype(np.float32)
         d = d[(d <= np.float32(1.2) * mx) & (d >= np.float32(0.8) * mn)]
         lk = np.zeros(len(d), np.int32); lf = np.zeros(len(d), np.int32); inv = np.zeros(2, np.float32)
-        L.ref_mp_predict_scale(C.c_float(mn), C.c_float(mx), d.ctypes.data_as(v), len(d), nlevels, C.c_float(log_sf), lk.ctypes.data_as(v), lf.ctypes.data_as(v), inv.ctypes.data_as(v))
+        L.ref_mp_predict_scale(C.c_float(mn), C.c_float(mx), RG.ptr(d), len(d), nlevels, C.c_float(log_sf), RG.ptr(lk), RG.ptr(lf), RG.ptr(inv))
         assert np.array_equal(lk, lf)
         assert inv[0] == np.float32(0.8) * mn and inv[1] == np.float32(1.2) * mx
         xyz = np.zeros((len(d), 3), np.float32); xyz[:, 2] = d

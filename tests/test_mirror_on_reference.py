@@ -73,7 +73,7 @@ def test_mirror_headers_inside_the_reference_tracking_thread(mirror_lib, seed, m
         for j in np.nonzero(lm['lid'][:m] >= 0)[0]:
             l = lm['lid'][j]
             lm['xyz'][l] = ti['lxyz'][f, j]; lm['obs'][l] = (ti['lflags'][f, j] >> 1) & 1; lm['valid'][l] = 0 if ti['lflags'][f, j] & 4 else 1
-        a = reference_chain(camv, sf, isig, cur, Tc[f], m, ti, f, lm, pc)                      # ORBmatcher.cc + Optimizer.cc + g2o
+        a = reference_chain(camv, sf, isig, cur, Tc[f], m, ti, f, lm, pc, lib=REFLIB)          # ORBmatcher.cc + Optimizer.cc + g2o
         b = reference_chain(camv, sf, isig, cur, Tc[f], m, ti, f, lm, pc, lib=mirror_lib)      # the mirror headers on the oracle-backed C ABI
         assert a['ok1'].value == b['ok1'].value and a['ok2'].value == b['ok2'].value and a['inl'].value == b['inl'].value, f
         assert np.array_equal(a['mp1'], b['mp1']) and np.array_equal(a['mp2'], b['mp2']) and np.array_equal(a['outl'], b['outl']), f

@@ -8,27 +8,25 @@ import ctypes as C
 import os
 
 import numpy as np
-import pytest
 
 import oracle as O
+import refgolden as RG
 import scenarios as S
 
 LIB = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'oracle', '_ref', 'liboptimizer_ref.so')
-pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason='oracle/_ref/liboptimizer_ref.so not built (reference tree absent)')
-v = C.c_void_p
 POSE_TOL = 1e-6
 
 
 def ref_pose_optimization(s):
-    L = C.CDLL(LIB); L.ref_pose_optimization.restype = C.c_int
+    L = RG.load(LIB, __name__); L.ref_pose_optimization.restype = C.c_int
     c = s['cam']; f32 = np.float32
     T = np.ascontiguousarray(s['T0'], f32).reshape(16)
     a = [np.ascontiguousarray(s['has'], np.uint8), np.ascontiguousarray(s['xyz'], f32), np.ascontiguousarray(s['xy'], f32), np.ascontiguousarray(s['octave'], np.int32),
          np.ascontiguousarray(s['uright'], f32)]
     isig = np.ascontiguousarray(s['inv_s2'], f32)
     n = len(a[0]); out = np.zeros(16, f32); outl = np.zeros(n, np.uint8)
-    r = L.ref_pose_optimization(T.ctypes.data_as(v), n, *[x.ctypes.data_as(v) for x in a], isig.ctypes.data_as(v), len(isig), C.c_float(c['fx']), C.c_float(c['fy']),
-                                C.c_float(c['cx']), C.c_float(c['cy']), C.c_float(c['bf']), out.ctypes.data_as(v), outl.ctypes.data_as(v))
+    r = L.ref_pose_optimization(RG.ptr(T), n, *[RG.ptr(x) for x in a], RG.ptr(isig), len(isig), C.c_float(c['fx']), C.c_float(c['fy']),
+                                C.c_float(c['cx']), C.c_float(c['cy']), C.c_float(c['bf']), RG.ptr(out), RG.ptr(outl))
     return r, out.reshape(4, 4), outl
 
 

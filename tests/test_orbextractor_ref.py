@@ -15,20 +15,19 @@ import numpy as np
 import pytest
 
 import oracle as O
+import refgolden as RG
 from pysgs import synth
 
 LIB = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'oracle', '_ref', 'liborbextractor_ref.so')
-pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason='oracle/_ref/liborbextractor_ref.so not built (reference tree absent)')
 
 
 def ref_extract(img, nfeatures=1000, scale=1.2, nlevels=8, ini=20, mn=7, monotone=True):
-    L = C.CDLL(LIB); L.ref_orb_extract.restype = C.c_int
+    L = RG.load(LIB, __name__); L.ref_orb_extract.restype = C.c_int
     L.ref_set_monotone_allocator(1 if monotone else 0)
     img = np.ascontiguousarray(img, np.uint8)
     cap = 4 * nfeatures + 4096
     k = np.zeros(cap, O.KP_DTYPE); d = np.zeros((cap, 32), np.uint8)
-    n = L.ref_orb_extract(img.ctypes.data_as(C.c_void_p), img.shape[1], img.shape[0], img.strides[0], nfeatures, C.c_float(scale), nlevels, ini, mn,
-                          k.ctypes.data_as(C.c_void_p), d.ctypes.data_as(C.c_void_p), cap)
+    n = L.ref_orb_extract(RG.ptr(img), img.shape[1], img.shape[0], img.strides[0], nfeatures, C.c_float(scale), nlevels, ini, mn, RG.ptr(k), RG.ptr(d), cap)
     L.ref_set_monotone_allocator(0)
     assert 0 <= n <= cap
     return k[:n], d[:n]

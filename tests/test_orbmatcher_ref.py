@@ -12,14 +12,14 @@ import numpy as np
 import pytest
 
 import oracle as O
+import refgolden as RG
 import scenarios as S
 
 LIB = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'oracle', '_ref', 'liborbmatcher_ref.so')
-pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason='oracle/_ref/liborbmatcher_ref.so not built (reference tree absent)')
 
 
 def _lib():
-    L = C.CDLL(LIB)
+    L = RG.load(LIB, __name__)
     L.ref_search_by_projection_last.restype = C.c_int
     L.ref_search_by_projection_local.restype = C.c_int
     L.ref_descriptor_distance.restype = C.c_int
@@ -27,7 +27,7 @@ def _lib():
 
 
 def _p(a):
-    return a.ctypes.data_as(C.c_void_p) if a is not None else None
+    return RG.ptr(a) if a is not None else None
 
 
 def _cam(s):

@@ -14,21 +14,20 @@ import numpy as np
 import pytest
 
 import oracle as O
+import refgolden as RG
 from pysgs import binding as B
 from pysgs import synth
 
 LIB = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'oracle', '_ref', 'libtracking_ref.so')
-pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason='oracle/_ref/libtracking_ref.so not built (reference tree absent)')
 W, H, TH = 640, 480, 15.0
-v = C.c_void_p
 
 
 def _p(a):
-    return a.ctypes.data_as(v)
+    return RG.ptr(a)
 
 
 def reference_chain(camv, sf, isig, cur, Tc, m, ti, f, lm, pc, lib=None):
-    L = C.CDLL(lib or LIB)
+    L = C.CDLL(lib) if lib else RG.load(LIB, __name__)
     n = cur.c.N
     xy = np.ascontiguousarray(np.stack([cur.keysUn['x'], cur.keysUn['y']], 1), np.float32)
     octv = np.ascontiguousarray(cur.keysUn['octave'], np.int32); ang = np.ascontiguousarray(cur.keysUn['angle'], np.float32)
