@@ -19,10 +19,8 @@
 #include <cstring>
 #include <vector>
 
+#include "host_call.h"
 #include "sgs_common.h"
-
-// host -> device copy of the convenience (host-pointer) entry points: the first failure is kept and reported by the caller
-#define SGS_H2D(err, dst, src, bytes) do { if ((err) == cudaSuccess) (err) = cudaMemcpy((dst), (src), (bytes), cudaMemcpyHostToDevice); } while (0)
 
 struct sgs_vocabulary {
     int device = 0, k = 0, L = 0, nnodes = 0;
@@ -454,24 +452,12 @@ SGS_API int sgs_bow_transform(const sgs_vocabulary* v, const uint8_t* desc, int 
     if (!v || n < 0 || (n > 0 && (!desc || !word || !weight || !node))) { set_error("sgs_bow_transform: bad argument"); return SGS_ERR_INVALID; }
     if (n == 0) return SGS_OK;
     SGS_CUDA_TRY(cudaSetDevice(v->device));
-    uint8_t* d = nullptr;
-    const size_t N = (size_t)n;
-    SGS_CUDA_TRY(cudaMalloc(&d, 32 * N + 8 * N + 4 * N + 4 * N + 64));
-    double* d_w = reinterpret_cast<double*>(d + 32 * N); int32_t* d_word = reinterpret_cast<int32_t*>(d_w + N); int32_t* d_node = d_word + N;
-    cudaError_t h2d = cudaSuccess;
-    SGS_H2D(h2d, d, desc, 32 * N);
-    if (h2d != cudaSuccess) { cudaFree(d); set_error("sgs_bow_transform: %s", cudaGetErrorString(h2d)); return SGS_ERR_CUDA; }
-    int rc = sgs_bow_transform_batch_device(v, d, nullptr, n, 1, levelsup, d_word, d_w, d_node, nullptr);
-    cudaError_t e = cudaSuccess;
-    if (rc == SGS_OK) {
-        e = cudaMemcpy(word, d_word, 4 * N, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(weight, d_w, 8 * N, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(node, d_node, 4 * N, cudaMemcpyDeviceToHost);
-    }
-    cudaFree(d);
-    if (rc != SGS_OK) return rc;
-    if (e != cudaSuccess) { set_error("sgs_bow_transform: %s", cudaGetErrorString(e)); return SGS_ERR_CUDA; }
-    return SGS_OK;
+    HostCall c("sgs_bow_transform");
+    const uint8_t* d_desc; int32_t *d_word, *d_node; double* d_weight;
+    c.in(&d_desc, desc, 32 * (size_t)n); c.out(&d_word, word, n); c.out(&d_weight, weight, n); c.out(&d_node, node, n);
+    if (int rc = c.upload()) return rc;
+    if (int rc = sgs_bow_transform_batch_device(v, d_desc, nullptr, n, 1, levelsup, d_word, d_weight, d_node, nullptr)) return rc;
+    return c.download();
 }
 
 SGS_API int sgs_match_bow(int nkf, const int32_t* kf_node, const double* kf_weight, const uint8_t* kf_valid, const uint8_t* kf_desc, const float* kf_angle,
@@ -483,41 +469,17 @@ SGS_API int sgs_match_bow(int nkf, const int32_t* kf_node, const double* kf_weig
     if (nkf == 0 || nf == 0) return SGS_OK;
     if (!kf_node || !kf_weight || !kf_valid || !kf_desc || !kf_angle || !f_node || !f_weight || !f_desc || !f_angle || !match_f) { set_error("sgs_match_bow: NULL array"); return SGS_ERR_INVALID; }
     SGS_CUDA_TRY(cudaSetDevice(device));
-    const size_t K = (size_t)nkf, F = (size_t)nf;
-    uint8_t* d = nullptr;
-    const size_t bytes = 8 * K + 8 * F + 32 * K + 32 * F + 4 * K + 4 * F + 4 * K + 4 * F + 4 * F + K + 64 + 16;
-    SGS_CUDA_TRY(cudaMalloc(&d, bytes));
-    double* d_kw = reinterpret_cast<double*>(d); double* d_fw = d_kw + K;
-    uint8_t* d_kd = reinterpret_cast<uint8_t*>(d_fw + F); uint8_t* d_fd = d_kd + 32 * K;
-    int32_t* d_kn = reinterpret_cast<int32_t*>(d_fd + 32 * F); int32_t* d_fn = d_kn + K;
-    float* d_ka = reinterpret_cast<float*>(d_fn + F); float* d_fa = d_ka + K;
-    int32_t* d_m = reinterpret_cast<int32_t*>(d_fa + F); int32_t* d_cnt = d_m + F;      // d_cnt: kf_n, f_n, nmatches
-    uint8_t* d_kv = reinterpret_cast<uint8_t*>(d_cnt + 4);
-    const int32_t cnt[3] = {nkf, nf, 0};
-    cudaError_t h2d = cudaSuccess;
-    SGS_H2D(h2d, d_kw, kf_weight, 8 * K); SGS_H2D(h2d, d_fw, f_weight, 8 * F);
-    SGS_H2D(h2d, d_kd, kf_desc, 32 * K); SGS_H2D(h2d, d_fd, f_desc, 32 * F);
-    SGS_H2D(h2d, d_kn, kf_node, 4 * K); SGS_H2D(h2d, d_fn, f_node, 4 * F);
-    SGS_H2D(h2d, d_ka, kf_angle, 4 * K); SGS_H2D(h2d, d_fa, f_angle, 4 * F);
-    SGS_H2D(h2d, d_kv, kf_valid, K); SGS_H2D(h2d, d_cnt, cnt, 12);
-    if (h2d != cudaSuccess) { cudaFree(d); set_error("sgs_match_bow: %s", cudaGetErrorString(h2d)); return SGS_ERR_CUDA; }
+    HostCall c("sgs_match_bow");
     sgs_bow_batch b;
     std::memset(&b, 0, sizeof b);
-    b.kf_node = d_kn; b.kf_weight = d_kw; b.kf_valid = d_kv; b.kf_desc = d_kd; b.kf_angle = d_ka; b.kf_n = d_cnt; b.kf_cap = nkf;
-    b.f_node = d_fn; b.f_weight = d_fw; b.f_desc = d_fd; b.f_angle = d_fa; b.f_n = d_cnt + 1; b.f_cap = nf;
-    b.nnratio = nnratio; b.check_orientation = check_orientation; b.match_f = d_m; b.nmatches = d_cnt + 2;
-    int rc = sgs_match_bow_batch_device(&b, 1, nullptr);
-    cudaError_t e = cudaSuccess;
-    int32_t nm = 0;
-    if (rc == SGS_OK) {
-        e = cudaMemcpy(match_f, d_m, 4 * F, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(&nm, d_cnt + 2, 4, cudaMemcpyDeviceToHost);
-    }
-    cudaFree(d);
-    if (rc != SGS_OK) return rc;
-    if (e != cudaSuccess) { set_error("sgs_match_bow: %s", cudaGetErrorString(e)); return SGS_ERR_CUDA; }
-    *nmatches = nm;
-    return SGS_OK;
+    c.in(&b.kf_node, kf_node, nkf); c.in(&b.kf_weight, kf_weight, nkf); c.in(&b.kf_valid, kf_valid, nkf); c.in(&b.kf_desc, kf_desc, 32 * (size_t)nkf);
+    c.in(&b.kf_angle, kf_angle, nkf); c.in(&b.kf_n, &nkf, 1);
+    c.in(&b.f_node, f_node, nf); c.in(&b.f_weight, f_weight, nf); c.in(&b.f_desc, f_desc, 32 * (size_t)nf); c.in(&b.f_angle, f_angle, nf); c.in(&b.f_n, &nf, 1);
+    c.out(&b.match_f, match_f, nf); c.out(&b.nmatches, nmatches, 1);
+    b.kf_cap = nkf; b.f_cap = nf; b.nnratio = nnratio; b.check_orientation = check_orientation;
+    if (int rc = c.upload()) return rc;
+    if (int rc = sgs_match_bow_batch_device(&b, 1, nullptr)) return rc;
+    return c.download();
 }
 
 }  // extern "C"

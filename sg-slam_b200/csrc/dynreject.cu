@@ -7,6 +7,7 @@
 
 #include <vector>
 
+#include "host_call.h"
 #include "sgs_common.h"
 
 namespace sgs {
@@ -126,21 +127,16 @@ SGS_API int sgs_dynreject(const float* cur_xy, const float* prev_xy, int n, cons
     *nkeep = n;
     if (restored) *restored = 0;
     SGS_CUDA_TRY(cudaSetDevice(device));
-    void *dc = nullptr, *dp = nullptr, *dF = nullptr, *db = nullptr, *dk = nullptr, *dd = nullptr;
-    struct Guard { void** p[6]; ~Guard() { for (auto q : p) if (*q) cudaFree(*q); } } guard{{&dc, &dp, &dF, &db, &dk, &dd}};
     if (n > 0) {
-        SGS_CUDA_TRY(cudaMalloc(&dc, 8 * (size_t)n)); SGS_CUDA_TRY(cudaMalloc(&dp, 8 * (size_t)n));
-        SGS_CUDA_TRY(cudaMalloc(&dF, 72)); SGS_CUDA_TRY(cudaMalloc(&db, sizeof(sgs_rect) * (size_t)(nboxes > 0 ? nboxes : 1)));
-        SGS_CUDA_TRY(cudaMalloc(&dk, n)); SGS_CUDA_TRY(cudaMalloc(&dd, 8 * (size_t)n));
-        SGS_CUDA_TRY(cudaMemcpy(dc, cur_xy, 8 * (size_t)n, cudaMemcpyHostToDevice));
-        SGS_CUDA_TRY(cudaMemcpy(dp, prev_xy, 8 * (size_t)n, cudaMemcpyHostToDevice));
-        if (F) SGS_CUDA_TRY(cudaMemcpy(dF, F, 72, cudaMemcpyHostToDevice));
-        if (nboxes) SGS_CUDA_TRY(cudaMemcpy(db, boxes, sizeof(sgs_rect) * nboxes, cudaMemcpyHostToDevice));
-        dynreject_flags_kernel<<<(n + 255) / 256, 256>>>((const float2*)dc, (const float2*)dp, n, (const double*)dF, F ? 1 : 0, (const sgs_rect*)db, nboxes,
-                                                         have_dyn, (uint8_t*)dk, (double*)dd);
+        HostCall c("sgs_dynreject");
+        const float2 *dc, *dp; const double* dF; const sgs_rect* db; uint8_t* dk; double* dd;
+        // without F or boxes the kernel reads neither, but still gets a valid address: that of an empty slice
+        c.in(&dc, cur_xy, n); c.in(&dp, prev_xy, n); c.in(&dF, F, F ? 9 : 0); c.in(&db, boxes, nboxes);
+        c.out(&dk, keep, n); c.out(&dd, dist, n);
+        if (int rc = c.upload()) return rc;
+        dynreject_flags_kernel<<<(n + 255) / 256, 256>>>(dc, dp, n, dF, F ? 1 : 0, db, nboxes, have_dyn, dk, dd);
         SGS_CUDA_TRY(cudaGetLastError());
-        SGS_CUDA_TRY(cudaMemcpy(keep, dk, n, cudaMemcpyDeviceToHost));
-        if (dist) SGS_CUDA_TRY(cudaMemcpy(dist, dd, 8 * (size_t)n, cudaMemcpyDeviceToHost));
+        if (int rc = c.download()) return rc;
     }
     int sum = 0;
     for (int i = 0; i < n; ++i) sum += keep[i];

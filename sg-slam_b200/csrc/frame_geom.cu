@@ -8,11 +8,9 @@
 // (device log vs glibc logf): the predicted level can differ when log(ratio)/log(scaleFactor) falls within an ulp of an integer.
 #include <cuda_runtime.h>
 
+#include "host_call.h"
 #include "sgs_common.h"
 #include "sgs_logf.h"
-
-// host -> device copy of the convenience (host-pointer) entry points: the first failure is kept and reported by the caller
-#define SGS_H2D(err, dst, src, bytes) do { if ((err) == cudaSuccess) (err) = cudaMemcpy((dst), (src), (bytes), cudaMemcpyHostToDevice); } while (0)
 
 namespace sgs {
 
@@ -143,17 +141,13 @@ SGS_API int sgs_undistort_points(const float* xy, int n, float fx, float fy, flo
     if (n < 0 || !dist_coef5 || (n > 0 && (!xy || !out_xy))) { set_error("sgs_undistort_points: bad argument"); return SGS_ERR_INVALID; }
     if (n == 0) return SGS_OK;
     SGS_CUDA_TRY(cudaSetDevice(device));
-    float2* d = nullptr;
-    SGS_CUDA_TRY(cudaMalloc(&d, 16 * (size_t)n));
-    cudaError_t h2d = cudaSuccess;
-    SGS_H2D(h2d, d, xy, 8 * (size_t)n);
-    if (h2d != cudaSuccess) { cudaFree(d); set_error("sgs_undistort_points: %s", cudaGetErrorString(h2d)); return SGS_ERR_CUDA; }
-    undistort_kernel<<<dim3((n + 255) / 256, 1), 256>>>(nullptr, d, nullptr, n, fx, fy, cx, cy, dist_coef5[0], dist_coef5[1], dist_coef5[2], dist_coef5[3],
-                                                        dist_coef5[4], nullptr, d + n);
-    cudaError_t e = cudaMemcpy(out_xy, d + n, 8 * (size_t)n, cudaMemcpyDeviceToHost);
-    cudaFree(d);
-    if (e != cudaSuccess) { set_error("sgs_undistort_points: %s", cudaGetErrorString(e)); return SGS_ERR_CUDA; }
-    return SGS_OK;
+    HostCall c("sgs_undistort_points");
+    const float2* d_xy; float2* d_out;
+    c.in(&d_xy, xy, n); c.out(&d_out, out_xy, n);
+    if (int rc = c.upload()) return rc;
+    undistort_kernel<<<dim3((n + 255) / 256, 1), 256>>>(nullptr, d_xy, nullptr, n, fx, fy, cx, cy, dist_coef5[0], dist_coef5[1], dist_coef5[2], dist_coef5[3],
+                                                        dist_coef5[4], nullptr, d_out);
+    return c.download();
 }
 
 // Frame::ComputeImageBounds (src/Frame.cc:686-714): mnMinX, mnMinY, mnMaxX, mnMaxY from the undistorted image corners
@@ -192,34 +186,16 @@ SGS_API int sgs_frustum(const sgs_camera* cam, const float* tcw, int n, const fl
     }
     if (n == 0) return SGS_OK;
     SGS_CUDA_TRY(cudaSetDevice(device));
-    // one allocation: inputs (16 + 8 n floats + 1 int) and outputs (4 n floats, n ints, n bytes)
-    const size_t N = (size_t)n;
-    float* d = nullptr;
-    SGS_CUDA_TRY(cudaMalloc(&d, sizeof(float) * (16 + 8 * N + 4 * N + N + 4) + N + 64));
-    float* d_tcw = d; float* d_xyz = d + 16; float* d_nrm = d_xyz + 3 * N; float* d_mn = d_nrm + 3 * N; float* d_mx = d_mn + N;
-    float* d_px = d_mx + N; float* d_py = d_px + N; float* d_pxr = d_py + N; float* d_vc = d_pxr + N;
-    int32_t* d_lv = reinterpret_cast<int32_t*>(d_vc + N); int32_t* d_n = d_lv + N; uint8_t* d_in = reinterpret_cast<uint8_t*>(d_n + 4);
-    cudaError_t h2d = cudaSuccess;
-    SGS_H2D(h2d, d_tcw, tcw, 64); SGS_H2D(h2d, d_xyz, xyz, 12 * N); SGS_H2D(h2d, d_nrm, normal, 12 * N);
-    SGS_H2D(h2d, d_mn, min_dist, 4 * N); SGS_H2D(h2d, d_mx, max_dist, 4 * N); SGS_H2D(h2d, d_n, &n, 4);
-    if (h2d != cudaSuccess) { cudaFree(d); set_error("sgs_frustum: %s", cudaGetErrorString(h2d)); return SGS_ERR_CUDA; }
+    HostCall c("sgs_frustum");
     sgs_frustum_batch a;
-    a.cam = *cam; a.tcw = d_tcw; a.mp_xyz = d_xyz; a.mp_normal = d_nrm; a.mp_min_dist = d_mn; a.mp_max_dist = d_mx; a.mp_n = d_n; a.point_cap = n;
-    a.viewing_cos_limit = viewing_cos_limit; a.mp_inview = d_in; a.proj_x = d_px; a.proj_y = d_py; a.proj_xr = d_pxr; a.level = d_lv; a.view_cos = d_vc;
-    int rc = sgs_frustum_batch_device(&a, 1, nullptr);
-    cudaError_t e = cudaSuccess;
-    if (rc == SGS_OK) {
-        e = cudaMemcpy(inview, d_in, N, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(proj_x, d_px, 4 * N, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(proj_y, d_py, 4 * N, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(proj_xr, d_pxr, 4 * N, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(view_cos, d_vc, 4 * N, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(level, d_lv, 4 * N, cudaMemcpyDeviceToHost);
-    }
-    cudaFree(d);
-    if (rc != SGS_OK) return rc;
-    if (e != cudaSuccess) { set_error("sgs_frustum: %s", cudaGetErrorString(e)); return SGS_ERR_CUDA; }
-    return SGS_OK;
+    c.in(&a.tcw, tcw, 16); c.in(&a.mp_xyz, xyz, 3 * (size_t)n); c.in(&a.mp_normal, normal, 3 * (size_t)n); c.in(&a.mp_min_dist, min_dist, n);
+    c.in(&a.mp_max_dist, max_dist, n); c.in(&a.mp_n, &n, 1);
+    c.out(&a.mp_inview, inview, n); c.out(&a.proj_x, proj_x, n); c.out(&a.proj_y, proj_y, n); c.out(&a.proj_xr, proj_xr, n); c.out(&a.view_cos, view_cos, n);
+    c.out(&a.level, level, n);
+    a.cam = *cam; a.point_cap = n; a.viewing_cos_limit = viewing_cos_limit;
+    if (int rc = c.upload()) return rc;
+    if (int rc = sgs_frustum_batch_device(&a, 1, nullptr)) return rc;
+    return c.download();
 }
 
 }  // extern "C"

@@ -17,10 +17,8 @@
 #include <cfloat>
 #include <vector>
 
+#include "host_call.h"
 #include "sgs_common.h"
-
-// host -> device copy of the convenience (host-pointer) entry points: the first failure is kept and reported by the caller
-#define SGS_H2D(err, dst, src, bytes) do { if ((err) == cudaSuccess) (err) = cudaMemcpy((dst), (src), (bytes), cudaMemcpyHostToDevice); } while (0)
 
 namespace sgs {
 
@@ -501,23 +499,13 @@ SGS_API int sgs_fundamental_ransac(const float* pts1_xy, const float* pts2_xy, i
                                    double* F, uint8_t* mask, int32_t* info, int device) {
     if (!pts1_xy || !pts2_xy || !F || n < 1) { set_error("sgs_fundamental_ransac: bad argument"); return SGS_ERR_INVALID; }
     SGS_CUDA_TRY(cudaSetDevice(device));
-    float* d_a = nullptr; float* d_b = nullptr; double* d_F = nullptr; int32_t* d_info = nullptr; uint8_t* d_mask = nullptr;
-    int rc = SGS_OK;
-    auto done = [&](int r) { cudaFree(d_a); cudaFree(d_b); cudaFree(d_F); cudaFree(d_info); cudaFree(d_mask); return r; };
-    SGS_CUDA_TRY(cudaMalloc(&d_a, 8 * (size_t)n));
-    if (cudaMalloc(&d_b, 8 * (size_t)n) != cudaSuccess || cudaMalloc(&d_F, 72) != cudaSuccess || cudaMalloc(&d_info, 16) != cudaSuccess ||
-        cudaMalloc(&d_mask, (size_t)n) != cudaSuccess) { set_error("sgs_fundamental_ransac: out of device memory"); return done(SGS_ERR_CUDA); }
-    cudaError_t h2d = cudaSuccess;
-    SGS_H2D(h2d, d_a, pts1_xy, 8 * (size_t)n); SGS_H2D(h2d, d_b, pts2_xy, 8 * (size_t)n);
-    if (h2d != cudaSuccess) { set_error("sgs_fundamental_ransac: %s", cudaGetErrorString(h2d)); return done(SGS_ERR_CUDA); }
-    rc = fm_launch(nullptr, reinterpret_cast<const float2*>(d_a), reinterpret_cast<const float2*>(d_b), nullptr, n, 1, nullptr, nullptr, nullptr, 0, nullptr,
-                   ransac_thresh, confidence, max_iters, d_F, d_info, d_mask, nullptr);
-    if (rc != SGS_OK) return done(rc);
-    cudaError_t e = cudaMemcpy(F, d_F, 72, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess && mask) e = cudaMemcpy(mask, d_mask, (size_t)n, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess && info) e = cudaMemcpy(info, d_info, 16, cudaMemcpyDeviceToHost);
-    if (e != cudaSuccess) { set_error("sgs_fundamental_ransac: %s", cudaGetErrorString(e)); return done(SGS_ERR_CUDA); }
-    return done(SGS_OK);
+    HostCall c("sgs_fundamental_ransac");
+    const float2 *d_a, *d_b; double* d_F; int32_t* d_info; uint8_t* d_mask;
+    c.in(&d_a, pts1_xy, n); c.in(&d_b, pts2_xy, n); c.out(&d_F, F, 9); c.out(&d_mask, mask, n); c.out(&d_info, info, 4);
+    if (int rc = c.upload()) return rc;
+    if (int rc = fm_launch(nullptr, d_a, d_b, nullptr, n, 1, nullptr, nullptr, nullptr, 0, nullptr, ransac_thresh, confidence, max_iters, d_F, d_info, d_mask, nullptr))
+        return rc;
+    return c.download();
 }
 
 }  // extern "C"

@@ -9,6 +9,7 @@
 
 #include <vector>
 
+#include "host_call.h"
 #include "sgs_common.h"
 
 namespace sgs {
@@ -101,29 +102,19 @@ int hamming_bf_device(const uint8_t* d_q, int nq, const uint8_t* d_t, int nt, in
 
 using namespace sgs;
 
-namespace {
-struct DevBuf {
-    void* p = nullptr;
-    ~DevBuf() { if (p) cudaFree(p); }
-    cudaError_t alloc(size_t bytes) { return cudaMalloc(&p, bytes ? bytes : 16); }
-    template <class T> T* as() { return static_cast<T*>(p); }
-};
-}  // namespace
-
 extern "C" {
 
 SGS_API int sgs_hamming_pairs(const uint8_t* a, const uint8_t* b, int n, int32_t* dist, int device) {
     if (n < 0 || (n > 0 && (!a || !b || !dist))) { set_error("sgs_hamming_pairs: bad argument"); return SGS_ERR_INVALID; }
     if (n == 0) return SGS_OK;
     SGS_CUDA_TRY(cudaSetDevice(device));
-    DevBuf da, db, dd;
-    SGS_CUDA_TRY(da.alloc((size_t)n * 32)); SGS_CUDA_TRY(db.alloc((size_t)n * 32)); SGS_CUDA_TRY(dd.alloc((size_t)n * 4));
-    SGS_CUDA_TRY(cudaMemcpy(da.p, a, (size_t)n * 32, cudaMemcpyHostToDevice));
-    SGS_CUDA_TRY(cudaMemcpy(db.p, b, (size_t)n * 32, cudaMemcpyHostToDevice));
-    hamming_pairs_kernel<<<(n + 255) / 256, 256>>>(da.as<uint4>(), db.as<uint4>(), n, dd.as<int32_t>());
+    HostCall c("sgs_hamming_pairs");
+    const uint4 *da, *db; int32_t* dd;
+    c.in(&da, a, 2 * (size_t)n); c.in(&db, b, 2 * (size_t)n); c.out(&dd, dist, n);
+    if (int rc = c.upload()) return rc;
+    hamming_pairs_kernel<<<(n + 255) / 256, 256>>>(da, db, n, dd);
     SGS_CUDA_TRY(cudaGetLastError());
-    SGS_CUDA_TRY(cudaMemcpy(dist, dd.p, (size_t)n * 4, cudaMemcpyDeviceToHost));
-    return SGS_OK;
+    return c.download();
 }
 
 SGS_API int sgs_hamming_bf_scratch_elems(int nq, int nt, int64_t* elems) {
@@ -150,18 +141,13 @@ SGS_API int sgs_hamming_bf(const uint8_t* query, int nq, const uint8_t* train, i
     if (!query || !best_idx || !best_dist || !second_dist || (nt > 0 && !train)) { set_error("sgs_hamming_bf: NULL pointer"); return SGS_ERR_INVALID; }
     SGS_CUDA_TRY(cudaSetDevice(device));
     const int ns = bf_plan_splits(nq, nt);
-    DevBuf dq, dt, di, dbst, dsec, dscr;
-    SGS_CUDA_TRY(dq.alloc((size_t)nq * 32)); SGS_CUDA_TRY(dt.alloc((size_t)nt * 32));
-    SGS_CUDA_TRY(di.alloc((size_t)nq * 4)); SGS_CUDA_TRY(dbst.alloc((size_t)nq * 4)); SGS_CUDA_TRY(dsec.alloc((size_t)nq * 4));
-    SGS_CUDA_TRY(dscr.alloc(ns > 1 ? (size_t)3 * ns * nq * 4 : 16));
-    SGS_CUDA_TRY(cudaMemcpy(dq.p, query, (size_t)nq * 32, cudaMemcpyHostToDevice));
-    if (nt) SGS_CUDA_TRY(cudaMemcpy(dt.p, train, (size_t)nt * 32, cudaMemcpyHostToDevice));
-    int rc = hamming_bf_device(dq.as<uint8_t>(), nq, dt.as<uint8_t>(), nt, di.as<int32_t>(), dbst.as<int32_t>(), dsec.as<int32_t>(), dscr.as<int32_t>(), ns, 0);
-    if (rc != SGS_OK) return rc;
-    SGS_CUDA_TRY(cudaMemcpy(best_idx, di.p, (size_t)nq * 4, cudaMemcpyDeviceToHost));
-    SGS_CUDA_TRY(cudaMemcpy(best_dist, dbst.p, (size_t)nq * 4, cudaMemcpyDeviceToHost));
-    SGS_CUDA_TRY(cudaMemcpy(second_dist, dsec.p, (size_t)nq * 4, cudaMemcpyDeviceToHost));
-    return SGS_OK;
+    HostCall c("sgs_hamming_bf");
+    const uint8_t *dq, *dt; int32_t *di, *dbst, *dsec, *dscr;
+    c.in(&dq, query, 32 * (size_t)nq); c.in(&dt, train, 32 * (size_t)nt);
+    c.out(&di, best_idx, nq); c.out(&dbst, best_dist, nq); c.out(&dsec, second_dist, nq); c.out(&dscr, nullptr, ns > 1 ? (size_t)3 * ns * nq : 0);
+    if (int rc = c.upload()) return rc;
+    if (int rc = hamming_bf_device(dq, nq, dt, nt, di, dbst, dsec, dscr, ns, 0)) return rc;
+    return c.download();
 }
 
 }  // extern "C"

@@ -5,6 +5,7 @@
 #include <cstring>
 #include <vector>
 
+#include "host_call.h"
 #include "match_dev.cuh"
 
 using namespace sgs;
@@ -28,18 +29,6 @@ MatchCam to_cam(const sgs_camera& c) {
     return m;
 }
 
-struct DevBuf {
-    void* p = nullptr;
-    ~DevBuf() { if (p) cudaFree(p); }
-    cudaError_t alloc(size_t bytes) { return cudaMalloc(&p, bytes ? bytes : 16); }
-    cudaError_t upload(const void* h, size_t bytes) {
-        cudaError_t e = alloc(bytes);
-        if (e != cudaSuccess || !bytes) return e;
-        return cudaMemcpy(p, h, bytes, cudaMemcpyHostToDevice);
-    }
-    template <class T> T* as() { return static_cast<T*>(p); }
-};
-
 sgs_camera view_cam(const sgs_frame_view* v) {
     sgs_camera c;
     std::memset(&c, 0, sizeof c);
@@ -49,13 +38,27 @@ sgs_camera view_cam(const sgs_frame_view* v) {
     return c;
 }
 
+int check_cur_cap(int cur_cap) {
+    if (cur_cap > 8192) { set_error("sgs_matcher_create: cur_cap %d exceeds the 8192 keypoints per frame the shared-memory grid supports", cur_cap); return SGS_ERR_UNSUPPORTED; }
+    return SGS_OK;
+}
+
+// the one-frame matcher of a host-pointer call: sgs_matcher_create(device, 1, cur_cap, point_cap), its scratch taken from the call's allocation
+int stage_matcher(HostCall& c, int device, int cur_cap, int point_cap, sgs_matcher* m) {
+    if (int rc = check_cur_cap(cur_cap)) return rc;
+    SGS_CUDA_TRY(cudaSetDevice(device));
+    m->device = device; m->max_frames = 1; m->cur_cap = cur_cap; m->point_cap = point_cap;
+    c.out(&m->d_pre, nullptr, point_cap); c.out(&m->d_lpre, nullptr, point_cap); c.out(&m->d_events, nullptr, point_cap);
+    return SGS_OK;
+}
+
 }  // namespace
 
 extern "C" {
 
 SGS_API int sgs_matcher_create(int device, int max_frames, int cur_cap, int point_cap, sgs_matcher** out) {
     if (!out || max_frames < 1 || cur_cap < 1 || point_cap < 1) { set_error("sgs_matcher_create: bad argument"); return SGS_ERR_INVALID; }
-    if (cur_cap > 8192) { set_error("sgs_matcher_create: cur_cap %d exceeds the 8192 keypoints per frame the shared-memory grid supports", cur_cap); return SGS_ERR_UNSUPPORTED; }
+    if (int rc = check_cur_cap(cur_cap)) return rc;
     *out = nullptr;
     SGS_CUDA_TRY(cudaSetDevice(device));
     sgs_matcher* m = new sgs_matcher();
@@ -160,40 +163,26 @@ SGS_API int sgs_match_project_lastframe(const sgs_frame_view* cur, const float* 
     if (!last_has_mp || !last_xyz || !last_desc || !last_obs || !last_octave || !last_angle || !cur_mp_inout || !cur->keys_un || !cur->u_right || !cur->desc) {
         set_error("sgs_match_project_lastframe: NULL array"); return SGS_ERR_INVALID;
     }
-    sgs_matcher* m = nullptr;
-    int rc = sgs_matcher_create(device, 1, cur->n, nlast, &m);
-    if (rc != SGS_OK) return rc;
-    struct Guard { sgs_matcher* m; ~Guard() { sgs_matcher_destroy(m); } } guard{m};
+    HostCall c("sgs_match_project_lastframe");
+    sgs_matcher m;
+    if (int rc = stage_matcher(c, device, cur->n, nlast, &m)) return rc;
     const int n = cur->n;
     std::vector<uint8_t> flags(nlast);
     for (int i = 0; i < nlast; ++i) flags[i] = (uint8_t)((last_has_mp[i] ? 1 : 0) | (last_obs[i] ? 2 : 0));
-    DevBuf kps, desc, ur, cn, xyz, ld, lf, lo, la, ln, tc, tl, mp, mpo, nm, nc;
-    const int32_t n32 = n, nl32 = nlast;
-    SGS_CUDA_TRY(kps.upload(cur->keys_un, sizeof(sgs_keypoint) * n)); SGS_CUDA_TRY(desc.upload(cur->desc, (size_t)32 * n));
-    SGS_CUDA_TRY(ur.upload(cur->u_right, 4 * (size_t)n)); SGS_CUDA_TRY(cn.upload(&n32, 4));
-    SGS_CUDA_TRY(xyz.upload(last_xyz, 12 * (size_t)nlast)); SGS_CUDA_TRY(ld.upload(last_desc, 32 * (size_t)nlast));
-    SGS_CUDA_TRY(lf.upload(flags.data(), nlast)); SGS_CUDA_TRY(lo.upload(last_octave, 4 * (size_t)nlast));
-    SGS_CUDA_TRY(la.upload(last_angle, 4 * (size_t)nlast)); SGS_CUDA_TRY(ln.upload(&nl32, 4));
-    SGS_CUDA_TRY(tc.upload(tcw_cur, 64)); SGS_CUDA_TRY(tl.upload(tcw_last, 64));
-    SGS_CUDA_TRY(mp.upload(cur_mp_inout, 4 * (size_t)n));
-    if (cur_mp_obs_in) SGS_CUDA_TRY(mpo.upload(cur_mp_obs_in, n));
-    SGS_CUDA_TRY(nm.alloc(4)); SGS_CUDA_TRY(nc.alloc(8)); SGS_CUDA_TRY(cudaMemset(nc.p, 0, 8));
     sgs_lastframe_batch b;
     std::memset(&b, 0, sizeof b);
     b.cam = view_cam(cur);
-    b.cur_kps = kps.as<sgs_keypoint>(); b.cur_desc = desc.as<uint8_t>(); b.cur_uright = ur.as<float>(); b.cur_n = cn.as<int32_t>();
-    b.last_xyz = xyz.as<float>(); b.last_desc = ld.as<uint8_t>(); b.last_flags = lf.as<uint8_t>(); b.last_octave = lo.as<int32_t>();
-    b.last_angle = la.as<float>(); b.last_n = ln.as<int32_t>(); b.tcw_cur = tc.as<float>(); b.tcw_last = tl.as<float>();
+    c.in(&b.cur_kps, cur->keys_un, n); c.in(&b.cur_desc, cur->desc, 32 * (size_t)n); c.in(&b.cur_uright, cur->u_right, n); c.in(&b.cur_n, &cur->n, 1);
+    c.in(&b.last_xyz, last_xyz, 3 * (size_t)nlast); c.in(&b.last_desc, last_desc, 32 * (size_t)nlast); c.in(&b.last_flags, flags.data(), nlast);
+    c.in(&b.last_octave, last_octave, nlast); c.in(&b.last_angle, last_angle, nlast); c.in(&b.last_n, &nlast, 1);
+    c.in(&b.tcw_cur, tcw_cur, 16); c.in(&b.tcw_last, tcw_last, 16);
+    c.inout(&b.cur_mp, cur_mp_inout, n);
+    if (cur_mp_obs_in) c.in(&b.cur_mp_obs_in, cur_mp_obs_in, n);
+    c.out(&b.nmatches, nmatches, 1); c.out(&b.ncand, nullptr, 1, true);
     b.th = th; b.mono = mono; b.check_orientation = check_orientation;
-    b.cur_mp = mp.as<int32_t>(); b.cur_mp_obs_in = cur_mp_obs_in ? mpo.as<uint8_t>() : nullptr; b.nmatches = nm.as<int32_t>(); b.ncand = nc.as<uint64_t>();
-    rc = sgs_match_project_lastframe_batch_device(m, &b, 1, nullptr);
-    if (rc != SGS_OK) return rc;
-    SGS_CUDA_TRY(cudaDeviceSynchronize());
-    int32_t nm_h = 0;
-    SGS_CUDA_TRY(cudaMemcpy(&nm_h, nm.p, 4, cudaMemcpyDeviceToHost));
-    SGS_CUDA_TRY(cudaMemcpy(cur_mp_inout, mp.p, 4 * (size_t)n, cudaMemcpyDeviceToHost));
-    *nmatches = nm_h;
-    return SGS_OK;
+    if (int rc = c.upload()) return rc;
+    if (int rc = sgs_match_project_lastframe_batch_device(&m, &b, 1, nullptr)) return rc;
+    return c.download();
 }
 
 SGS_API int sgs_match_project_keyframe(const sgs_frame_view* cur, const float* tcw_cur, int nkf, const uint8_t* kf_valid, const float* kf_xyz,
@@ -205,37 +194,24 @@ SGS_API int sgs_match_project_keyframe(const sgs_frame_view* cur, const float* t
     if (!kf_valid || !kf_xyz || !kf_desc || !kf_angle || !kf_min_dist || !kf_max_dist || !cur_mp_inout || !cur->keys_un || !cur->u_right || !cur->desc) {
         set_error("sgs_match_project_keyframe: NULL array"); return SGS_ERR_INVALID;
     }
-    sgs_matcher* m = nullptr;
-    int rc = sgs_matcher_create(device, 1, cur->n, nkf, &m);
-    if (rc != SGS_OK) return rc;
-    struct Guard { sgs_matcher* m; ~Guard() { sgs_matcher_destroy(m); } } guard{m};
+    HostCall c("sgs_match_project_keyframe");
+    sgs_matcher m;
+    if (int rc = stage_matcher(c, device, cur->n, nkf, &m)) return rc;
     const int n = cur->n;
-    const int32_t n32 = n, nkf32 = nkf;
     std::vector<uint8_t> flags(nkf);
     for (int i = 0; i < nkf; ++i) flags[i] = kf_valid[i] ? 1 : 0;
-    DevBuf kps, desc, ur, cn, fl, xyz, kd, ang, mn, mx, kn, tc, mp, nm, nc;
-    SGS_CUDA_TRY(kps.upload(cur->keys_un, sizeof(sgs_keypoint) * n)); SGS_CUDA_TRY(desc.upload(cur->desc, (size_t)32 * n));
-    SGS_CUDA_TRY(ur.upload(cur->u_right, 4 * (size_t)n)); SGS_CUDA_TRY(cn.upload(&n32, 4));
-    SGS_CUDA_TRY(fl.upload(flags.data(), nkf)); SGS_CUDA_TRY(xyz.upload(kf_xyz, 12 * (size_t)nkf)); SGS_CUDA_TRY(kd.upload(kf_desc, 32 * (size_t)nkf));
-    SGS_CUDA_TRY(ang.upload(kf_angle, 4 * (size_t)nkf)); SGS_CUDA_TRY(mn.upload(kf_min_dist, 4 * (size_t)nkf)); SGS_CUDA_TRY(mx.upload(kf_max_dist, 4 * (size_t)nkf));
-    SGS_CUDA_TRY(kn.upload(&nkf32, 4)); SGS_CUDA_TRY(tc.upload(tcw_cur, 64)); SGS_CUDA_TRY(mp.upload(cur_mp_inout, 4 * (size_t)n));
-    SGS_CUDA_TRY(nm.alloc(4)); SGS_CUDA_TRY(nc.alloc(8)); SGS_CUDA_TRY(cudaMemset(nc.p, 0, 8));
     sgs_keyframe_batch b;
     std::memset(&b, 0, sizeof b);
     b.cam = view_cam(cur);
-    b.cur_kps = kps.as<sgs_keypoint>(); b.cur_desc = desc.as<uint8_t>(); b.cur_uright = ur.as<float>(); b.cur_n = cn.as<int32_t>();
-    b.kf_xyz = xyz.as<float>(); b.kf_desc = kd.as<uint8_t>(); b.kf_valid = fl.as<uint8_t>(); b.kf_angle = ang.as<float>();
-    b.kf_min_dist = mn.as<float>(); b.kf_max_dist = mx.as<float>(); b.kf_n = kn.as<int32_t>(); b.tcw_cur = tc.as<float>();
+    c.in(&b.cur_kps, cur->keys_un, n); c.in(&b.cur_desc, cur->desc, 32 * (size_t)n); c.in(&b.cur_uright, cur->u_right, n); c.in(&b.cur_n, &cur->n, 1);
+    c.in(&b.kf_valid, flags.data(), nkf); c.in(&b.kf_xyz, kf_xyz, 3 * (size_t)nkf); c.in(&b.kf_desc, kf_desc, 32 * (size_t)nkf);
+    c.in(&b.kf_angle, kf_angle, nkf); c.in(&b.kf_min_dist, kf_min_dist, nkf); c.in(&b.kf_max_dist, kf_max_dist, nkf);
+    c.in(&b.kf_n, &nkf, 1); c.in(&b.tcw_cur, tcw_cur, 16);
+    c.inout(&b.cur_mp, cur_mp_inout, n); c.out(&b.nmatches, nmatches, 1); c.out(&b.ncand, nullptr, 1, true);
     b.th = th; b.orb_dist = orb_dist; b.check_orientation = check_orientation;
-    b.cur_mp = mp.as<int32_t>(); b.nmatches = nm.as<int32_t>(); b.ncand = nc.as<uint64_t>();
-    rc = sgs_match_project_keyframe_batch_device(m, &b, 1, nullptr);
-    if (rc != SGS_OK) return rc;
-    SGS_CUDA_TRY(cudaDeviceSynchronize());
-    int32_t nm_h = 0;
-    SGS_CUDA_TRY(cudaMemcpy(&nm_h, nm.p, 4, cudaMemcpyDeviceToHost));
-    SGS_CUDA_TRY(cudaMemcpy(cur_mp_inout, mp.p, 4 * (size_t)n, cudaMemcpyDeviceToHost));
-    *nmatches = nm_h;
-    return SGS_OK;
+    if (int rc = c.upload()) return rc;
+    if (int rc = sgs_match_project_keyframe_batch_device(&m, &b, 1, nullptr)) return rc;
+    return c.download();
 }
 
 SGS_API int sgs_fuse_search(const sgs_frame_view* kf, const float* tcw, const float* ow, int nmp, const uint8_t* mp_valid, const float* mp_xyz,
@@ -250,36 +226,24 @@ SGS_API int sgs_fuse_search(const sgs_frame_view* kf, const float* tcw, const fl
         (sim3_variant == 0 && !inv_level_sigma2) || (sim3_variant == 3 && !kf_matched_inout)) { set_error("sgs_fuse_search: NULL array"); return SGS_ERR_INVALID; }
     SGS_CUDA_TRY(cudaSetDevice(device));
     const int n = kf->n;
-    const int32_t n32 = n, nmp32 = nmp;
-    DevBuf kps, desc, ur, kn, tc, o, xyz, nrm, mn, mx, md, mv, mpn, xf, bi, bd, km, nm;
-    SGS_CUDA_TRY(kps.upload(kf->keys_un, sizeof(sgs_keypoint) * n)); SGS_CUDA_TRY(desc.upload(kf->desc, (size_t)32 * n)); SGS_CUDA_TRY(ur.upload(kf->u_right, 4 * (size_t)n));
-    SGS_CUDA_TRY(kn.upload(&n32, 4)); SGS_CUDA_TRY(tc.upload(tcw, 64)); SGS_CUDA_TRY(o.upload(ow, 12));
-    SGS_CUDA_TRY(xyz.upload(mp_xyz, 12 * (size_t)nmp)); SGS_CUDA_TRY(nrm.upload(mp_normal, 12 * (size_t)nmp)); SGS_CUDA_TRY(mn.upload(mp_min_dist, 4 * (size_t)nmp));
-    SGS_CUDA_TRY(mx.upload(mp_max_dist, 4 * (size_t)nmp)); SGS_CUDA_TRY(md.upload(mp_desc, 32 * (size_t)nmp)); SGS_CUDA_TRY(mv.upload(mp_valid, (size_t)nmp));
-    SGS_CUDA_TRY(mpn.upload(&nmp32, 4)); SGS_CUDA_TRY(bi.alloc(4 * (size_t)nmp)); SGS_CUDA_TRY(bd.alloc(4 * (size_t)nmp)); SGS_CUDA_TRY(nm.alloc(4));
-    if (xform2) SGS_CUDA_TRY(xf.upload(xform2, 48));
-    if (kf_matched_inout) SGS_CUDA_TRY(km.upload(kf_matched_inout, 4 * (size_t)n));
+    HostCall c("sgs_fuse_search");
     sgs_fuse_batch b;
     std::memset(&b, 0, sizeof b);
     b.cam = view_cam(kf);
-    b.kf_kps = kps.as<sgs_keypoint>(); b.kf_desc = desc.as<uint8_t>(); b.kf_uright = ur.as<float>(); b.kf_n = kn.as<int32_t>(); b.kf_cap = n;
-    b.tcw = tc.as<float>(); b.ow = o.as<float>(); b.mp_xyz = xyz.as<float>(); b.mp_normal = nrm.as<float>(); b.mp_min_dist = mn.as<float>(); b.mp_max_dist = mx.as<float>();
-    b.mp_desc = md.as<uint8_t>(); b.mp_valid = mv.as<uint8_t>(); b.mp_n = mpn.as<int32_t>(); b.mp_cap = nmp; b.th = th;
+    c.in(&b.kf_kps, kf->keys_un, n); c.in(&b.kf_desc, kf->desc, 32 * (size_t)n); c.in(&b.kf_uright, kf->u_right, n); c.in(&b.kf_n, &kf->n, 1);
+    c.in(&b.tcw, tcw, 16); c.in(&b.ow, ow, 3);
+    c.in(&b.mp_xyz, mp_xyz, 3 * (size_t)nmp); c.in(&b.mp_normal, mp_normal, 3 * (size_t)nmp); c.in(&b.mp_min_dist, mp_min_dist, nmp);
+    c.in(&b.mp_max_dist, mp_max_dist, nmp); c.in(&b.mp_desc, mp_desc, 32 * (size_t)nmp); c.in(&b.mp_valid, mp_valid, nmp); c.in(&b.mp_n, &nmp, 1);
+    if (xform2) c.in(&b.xform2, xform2, 12);
+    c.out(&b.best_idx, best_idx, nmp); c.out(&b.best_dist, best_dist, nmp);
+    // vpMatched and the match count belong to variant 3 alone: only it reads and writes them, and only it copies them back
+    if (sim3_variant == 3) c.inout(&b.kf_matched, kf_matched_inout, n);
+    c.out(&b.nmatches, sim3_variant == 3 ? nmatches : nullptr, 1);
+    b.kf_cap = n; b.mp_cap = nmp; b.th = th; b.sim3_variant = sim3_variant;
     for (int l = 0; l < 16; ++l) b.inv_level_sigma2[l] = inv_level_sigma2 && l < kf->nlevels ? inv_level_sigma2[l] : 0.f;
-    b.sim3_variant = sim3_variant; b.xform2 = xform2 ? xf.as<float>() : nullptr;
-    b.best_idx = bi.as<int32_t>(); b.best_dist = bd.as<int32_t>(); b.kf_matched = kf_matched_inout ? km.as<int32_t>() : nullptr; b.nmatches = nm.as<int32_t>();
-    const int rc = sgs_fuse_search_batch_device(&b, 1, nullptr);
-    if (rc != SGS_OK) return rc;
-    SGS_CUDA_TRY(cudaDeviceSynchronize());
-    SGS_CUDA_TRY(cudaMemcpy(best_idx, bi.p, 4 * (size_t)nmp, cudaMemcpyDeviceToHost));
-    SGS_CUDA_TRY(cudaMemcpy(best_dist, bd.p, 4 * (size_t)nmp, cudaMemcpyDeviceToHost));
-    if (sim3_variant == 3) {
-        SGS_CUDA_TRY(cudaMemcpy(kf_matched_inout, km.p, 4 * (size_t)n, cudaMemcpyDeviceToHost));
-        int32_t nm_h = 0;
-        SGS_CUDA_TRY(cudaMemcpy(&nm_h, nm.p, 4, cudaMemcpyDeviceToHost));
-        if (nmatches) *nmatches = nm_h;
-    }
-    return SGS_OK;
+    if (int rc = c.upload()) return rc;
+    if (int rc = sgs_fuse_search_batch_device(&b, 1, nullptr)) return rc;
+    return c.download();
 }
 
 SGS_API int sgs_search_for_initialization_batch_device(const sgs_init_batch* a, int nframes, void* stream) {
@@ -301,28 +265,17 @@ SGS_API int sgs_search_for_initialization(const sgs_frame_view* f1, const sgs_fr
     if (f1->n == 0 || f2->n == 0) return SGS_OK;
     if (!prev_xy || !match12 || !f1->keys_un || !f1->desc || !f2->keys_un || !f2->desc) { set_error("sgs_search_for_initialization: NULL array"); return SGS_ERR_INVALID; }
     SGS_CUDA_TRY(cudaSetDevice(device));
-    const size_t A1 = (size_t)f1->n, A2 = (size_t)f2->n;
-    const int32_t cnt[3] = {f1->n, f2->n, 0};
-    DevBuf k1, d1, k2, d2, c, pv, m;
-    SGS_CUDA_TRY(k1.upload(f1->keys_un, sizeof(sgs_keypoint) * A1)); SGS_CUDA_TRY(d1.upload(f1->desc, 32 * A1));
-    SGS_CUDA_TRY(k2.upload(f2->keys_un, sizeof(sgs_keypoint) * A2)); SGS_CUDA_TRY(d2.upload(f2->desc, 32 * A2));
-    SGS_CUDA_TRY(c.upload(cnt, 12)); SGS_CUDA_TRY(pv.upload(prev_xy, 8 * A1)); SGS_CUDA_TRY(m.alloc(4 * A1));
+    HostCall c("sgs_search_for_initialization");
     sgs_init_batch b;
     std::memset(&b, 0, sizeof b);
     b.cam = view_cam(f2);
-    b.f1_kps = k1.as<sgs_keypoint>(); b.f1_desc = d1.as<uint8_t>(); b.f1_n = c.as<int32_t>(); b.f1_cap = f1->n;
-    b.f2_kps = k2.as<sgs_keypoint>(); b.f2_desc = d2.as<uint8_t>(); b.f2_n = c.as<int32_t>() + 1; b.f2_cap = f2->n;
-    b.prev_xy = pv.as<float>(); b.window_size = window_size; b.nnratio = nnratio; b.check_orientation = check_orientation;
-    b.match12 = m.as<int32_t>(); b.nmatches = c.as<int32_t>() + 2;
-    const int rc = sgs_search_for_initialization_batch_device(&b, 1, nullptr);
-    if (rc != SGS_OK) return rc;
-    SGS_CUDA_TRY(cudaDeviceSynchronize());
-    SGS_CUDA_TRY(cudaMemcpy(match12, m.p, 4 * A1, cudaMemcpyDeviceToHost));
-    SGS_CUDA_TRY(cudaMemcpy(prev_xy, pv.p, 8 * A1, cudaMemcpyDeviceToHost));
-    int32_t nm = 0;
-    SGS_CUDA_TRY(cudaMemcpy(&nm, c.as<int32_t>() + 2, 4, cudaMemcpyDeviceToHost));
-    *nmatches = nm;
-    return SGS_OK;
+    c.in(&b.f1_kps, f1->keys_un, f1->n); c.in(&b.f1_desc, f1->desc, 32 * (size_t)f1->n); c.in(&b.f1_n, &f1->n, 1);
+    c.in(&b.f2_kps, f2->keys_un, f2->n); c.in(&b.f2_desc, f2->desc, 32 * (size_t)f2->n); c.in(&b.f2_n, &f2->n, 1);
+    c.inout(&b.prev_xy, prev_xy, 2 * (size_t)f1->n); c.out(&b.match12, match12, f1->n); c.out(&b.nmatches, nmatches, 1);
+    b.f1_cap = f1->n; b.f2_cap = f2->n; b.window_size = window_size; b.nnratio = nnratio; b.check_orientation = check_orientation;
+    if (int rc = c.upload()) return rc;
+    if (int rc = sgs_search_for_initialization_batch_device(&b, 1, nullptr)) return rc;
+    return c.download();
 }
 
 SGS_API int sgs_match_bow_keyframes(int mode, int n1, const int32_t* node1, const double* weight1, const uint8_t* valid1, const uint8_t* desc1, const float* angle1,
@@ -338,32 +291,22 @@ SGS_API int sgs_match_bow_keyframes(int mode, int n1, const int32_t* node1, cons
     if (mode == 2 && (!stereo1 || !stereo2 || !xy1 || !xy2 || !octave2 || !F12 || !epipole || !level_sigma2 || !scale_factors || nlevels < 1 || nlevels > 16)) {
         set_error("sgs_match_bow_keyframes: triangulation mode needs stereo flags, positions, octaves, F12, the epipole and the level tables"); return SGS_ERR_INVALID; }
     SGS_CUDA_TRY(cudaSetDevice(device));
-    const size_t A = (size_t)n1, Bn = (size_t)n2;
-    const int32_t cnt[3] = {n1, n2, 0};
-    DevBuf nd1, w1, v1, d1, a1, nd2, w2, v2, d2, a2, c, m, s1, s2, p1, p2, o2, f, ep;
-    SGS_CUDA_TRY(nd1.upload(node1, 4 * A)); SGS_CUDA_TRY(w1.upload(weight1, 8 * A)); SGS_CUDA_TRY(v1.upload(valid1, A)); SGS_CUDA_TRY(d1.upload(desc1, 32 * A)); SGS_CUDA_TRY(a1.upload(angle1, 4 * A));
-    SGS_CUDA_TRY(nd2.upload(node2, 4 * Bn)); SGS_CUDA_TRY(w2.upload(weight2, 8 * Bn)); SGS_CUDA_TRY(v2.upload(valid2, Bn)); SGS_CUDA_TRY(d2.upload(desc2, 32 * Bn)); SGS_CUDA_TRY(a2.upload(angle2, 4 * Bn));
-    SGS_CUDA_TRY(c.upload(cnt, 12)); SGS_CUDA_TRY(m.alloc(4 * A));
+    HostCall c("sgs_match_bow_keyframes");
     sgs_bow_batch b;
     std::memset(&b, 0, sizeof b);
-    b.kf_node = nd1.as<int32_t>(); b.kf_weight = w1.as<double>(); b.kf_valid = v1.as<uint8_t>(); b.kf_desc = d1.as<uint8_t>(); b.kf_angle = a1.as<float>(); b.kf_n = c.as<int32_t>(); b.kf_cap = n1;
-    b.f_node = nd2.as<int32_t>(); b.f_weight = w2.as<double>(); b.f_valid = v2.as<uint8_t>(); b.f_desc = d2.as<uint8_t>(); b.f_angle = a2.as<float>(); b.f_n = c.as<int32_t>() + 1; b.f_cap = n2;
-    b.keyframe_pair = mode; b.nnratio = nnratio; b.check_orientation = check_orientation; b.match_f = m.as<int32_t>(); b.nmatches = c.as<int32_t>() + 2;
+    c.in(&b.kf_node, node1, n1); c.in(&b.kf_weight, weight1, n1); c.in(&b.kf_valid, valid1, n1); c.in(&b.kf_desc, desc1, 32 * (size_t)n1); c.in(&b.kf_angle, angle1, n1);
+    c.in(&b.f_node, node2, n2); c.in(&b.f_weight, weight2, n2); c.in(&b.f_valid, valid2, n2); c.in(&b.f_desc, desc2, 32 * (size_t)n2); c.in(&b.f_angle, angle2, n2);
+    c.in(&b.kf_n, &n1, 1); c.in(&b.f_n, &n2, 1); c.out(&b.match_f, match12, n1); c.out(&b.nmatches, nmatches, 1);
+    b.kf_cap = n1; b.f_cap = n2; b.keyframe_pair = mode; b.nnratio = nnratio; b.check_orientation = check_orientation;
     if (mode == 2) {
-        SGS_CUDA_TRY(s1.upload(stereo1, A)); SGS_CUDA_TRY(s2.upload(stereo2, Bn)); SGS_CUDA_TRY(p1.upload(xy1, 8 * A)); SGS_CUDA_TRY(p2.upload(xy2, 8 * Bn));
-        SGS_CUDA_TRY(o2.upload(octave2, 4 * Bn)); SGS_CUDA_TRY(f.upload(F12, 36)); SGS_CUDA_TRY(ep.upload(epipole, 8));
-        b.kf_stereo = s1.as<uint8_t>(); b.f_stereo = s2.as<uint8_t>(); b.kf_xy = p1.as<float>(); b.f_xy = p2.as<float>(); b.f_octave = o2.as<int32_t>();
-        b.F12 = f.as<float>(); b.epipole = ep.as<float>(); b.only_stereo = only_stereo;
+        c.in(&b.kf_stereo, stereo1, n1); c.in(&b.f_stereo, stereo2, n2); c.in(&b.kf_xy, xy1, 2 * (size_t)n1); c.in(&b.f_xy, xy2, 2 * (size_t)n2);
+        c.in(&b.f_octave, octave2, n2); c.in(&b.F12, F12, 9); c.in(&b.epipole, epipole, 2);
+        b.only_stereo = only_stereo;
         for (int l = 0; l < nlevels; ++l) { b.level_sigma2[l] = level_sigma2[l]; b.scale_factors[l] = scale_factors[l]; }
     }
-    const int rc = sgs_match_bow_batch_device(&b, 1, nullptr);
-    if (rc != SGS_OK) return rc;
-    SGS_CUDA_TRY(cudaDeviceSynchronize());
-    SGS_CUDA_TRY(cudaMemcpy(match12, m.p, 4 * A, cudaMemcpyDeviceToHost));
-    int32_t nm = 0;
-    SGS_CUDA_TRY(cudaMemcpy(&nm, c.as<int32_t>() + 2, 4, cudaMemcpyDeviceToHost));
-    *nmatches = nm;
-    return SGS_OK;
+    if (int rc = c.upload()) return rc;
+    if (int rc = sgs_match_bow_batch_device(&b, 1, nullptr)) return rc;
+    return c.download();
 }
 
 SGS_API int sgs_match_project_localmap(const sgs_frame_view* f, int nmp, const uint8_t* mp_inview, const float* proj_x, const float* proj_y,
@@ -376,37 +319,21 @@ SGS_API int sgs_match_project_localmap(const sgs_frame_view* f, int nmp, const u
     if (!mp_inview || !proj_x || !proj_y || !proj_xr || !level || !view_cos || !mp_desc || !mp_obs || !f_mp_inout || !f_mp_obs_inout) {
         set_error("sgs_match_project_localmap: NULL array"); return SGS_ERR_INVALID;
     }
-    sgs_matcher* m = nullptr;
-    int rc = sgs_matcher_create(device, 1, f->n, nmp, &m);
-    if (rc != SGS_OK) return rc;
-    struct Guard { sgs_matcher* m; ~Guard() { sgs_matcher_destroy(m); } } guard{m};
+    HostCall c("sgs_match_project_localmap");
+    sgs_matcher m;
+    if (int rc = stage_matcher(c, device, f->n, nmp, &m)) return rc;
     const int n = f->n;
-    const int32_t n32 = n, nmp32 = nmp;
-    DevBuf kps, desc, ur, cn, iv, px, py, pxr, lv, vc, md, mo, mn, mp, mpo, nm, nc;
-    SGS_CUDA_TRY(kps.upload(f->keys_un, sizeof(sgs_keypoint) * n)); SGS_CUDA_TRY(desc.upload(f->desc, (size_t)32 * n));
-    SGS_CUDA_TRY(ur.upload(f->u_right, 4 * (size_t)n)); SGS_CUDA_TRY(cn.upload(&n32, 4));
-    SGS_CUDA_TRY(iv.upload(mp_inview, nmp)); SGS_CUDA_TRY(px.upload(proj_x, 4 * (size_t)nmp)); SGS_CUDA_TRY(py.upload(proj_y, 4 * (size_t)nmp));
-    SGS_CUDA_TRY(pxr.upload(proj_xr, 4 * (size_t)nmp)); SGS_CUDA_TRY(lv.upload(level, 4 * (size_t)nmp)); SGS_CUDA_TRY(vc.upload(view_cos, 4 * (size_t)nmp));
-    SGS_CUDA_TRY(md.upload(mp_desc, 32 * (size_t)nmp)); SGS_CUDA_TRY(mo.upload(mp_obs, nmp)); SGS_CUDA_TRY(mn.upload(&nmp32, 4));
-    SGS_CUDA_TRY(mp.upload(f_mp_inout, 4 * (size_t)n)); SGS_CUDA_TRY(mpo.upload(f_mp_obs_inout, n));
-    SGS_CUDA_TRY(nm.alloc(4)); SGS_CUDA_TRY(nc.alloc(8)); SGS_CUDA_TRY(cudaMemset(nc.p, 0, 8));
     sgs_localmap_batch b;
     std::memset(&b, 0, sizeof b);
     b.cam = view_cam(f);
-    b.cur_kps = kps.as<sgs_keypoint>(); b.cur_desc = desc.as<uint8_t>(); b.cur_uright = ur.as<float>(); b.cur_n = cn.as<int32_t>();
-    b.mp_inview = iv.as<uint8_t>(); b.proj_x = px.as<float>(); b.proj_y = py.as<float>(); b.proj_xr = pxr.as<float>(); b.level = lv.as<int32_t>();
-    b.view_cos = vc.as<float>(); b.mp_desc = md.as<uint8_t>(); b.mp_obs = mo.as<uint8_t>(); b.mp_n = mn.as<int32_t>();
+    c.in(&b.cur_kps, f->keys_un, n); c.in(&b.cur_desc, f->desc, 32 * (size_t)n); c.in(&b.cur_uright, f->u_right, n); c.in(&b.cur_n, &f->n, 1);
+    c.in(&b.mp_inview, mp_inview, nmp); c.in(&b.proj_x, proj_x, nmp); c.in(&b.proj_y, proj_y, nmp); c.in(&b.proj_xr, proj_xr, nmp); c.in(&b.level, level, nmp);
+    c.in(&b.view_cos, view_cos, nmp); c.in(&b.mp_desc, mp_desc, 32 * (size_t)nmp); c.in(&b.mp_obs, mp_obs, nmp); c.in(&b.mp_n, &nmp, 1);
+    c.inout(&b.f_mp, f_mp_inout, n); c.inout(&b.f_mp_obs, f_mp_obs_inout, n); c.out(&b.nmatches, nmatches, 1); c.out(&b.ncand, nullptr, 1, true);
     b.th = th; b.nnratio = nnratio; b.id_base = id_base;
-    b.f_mp = mp.as<int32_t>(); b.f_mp_obs = mpo.as<uint8_t>(); b.nmatches = nm.as<int32_t>(); b.ncand = nc.as<uint64_t>();
-    rc = sgs_match_project_localmap_batch_device(m, &b, 1, nullptr);
-    if (rc != SGS_OK) return rc;
-    SGS_CUDA_TRY(cudaDeviceSynchronize());
-    int32_t nm_h = 0;
-    SGS_CUDA_TRY(cudaMemcpy(&nm_h, nm.p, 4, cudaMemcpyDeviceToHost));
-    SGS_CUDA_TRY(cudaMemcpy(f_mp_inout, mp.p, 4 * (size_t)n, cudaMemcpyDeviceToHost));
-    SGS_CUDA_TRY(cudaMemcpy(f_mp_obs_inout, mpo.p, n, cudaMemcpyDeviceToHost));
-    *nmatches = nm_h;
-    return SGS_OK;
+    if (int rc = c.upload()) return rc;
+    if (int rc = sgs_match_project_localmap_batch_device(&m, &b, 1, nullptr)) return rc;
+    return c.download();
 }
 
 }  // extern "C"

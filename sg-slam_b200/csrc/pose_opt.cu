@@ -12,6 +12,7 @@
 
 #include <cfloat>
 
+#include "host_call.h"
 #include "sgs_common.h"
 
 namespace sgs {
@@ -348,39 +349,18 @@ SGS_API int sgs_pose_optimization(const sgs_camera* cam, const float* tcw_in, in
     *ninliers = 0;
     if (n == 0) return SGS_OK;
     SGS_CUDA_TRY(cudaSetDevice(device));
-    const size_t N = (size_t)n;
-    uint8_t* d = nullptr;
-    const size_t bytes = 24 * N + sizeof(sgs_keypoint) * N + 4 * N + 12 * N + 64 + 64 + 16 + N + N + N + 256;
-    SGS_CUDA_TRY(cudaMalloc(&d, bytes));
-    double* d_err = reinterpret_cast<double*>(d);
-    sgs_keypoint* d_k = reinterpret_cast<sgs_keypoint*>(d_err + 3 * N);
-    float* d_ur = reinterpret_cast<float*>(d_k + N); float* d_xyz = d_ur + N; float* d_Tin = d_xyz + 3 * N; float* d_Tout = d_Tin + 16;
-    int32_t* d_n = reinterpret_cast<int32_t*>(d_Tout + 16); int32_t* d_nin = d_n + 1;
-    uint8_t* d_has = reinterpret_cast<uint8_t*>(d_n + 4); uint8_t* d_out = d_has + N; uint8_t* d_lvl = d_out + N;
-    cudaError_t e = cudaSuccess;
-    auto up = [&](void* dst, const void* src, size_t b) { if (e == cudaSuccess) e = cudaMemcpy(dst, src, b, cudaMemcpyHostToDevice); };
-    up(d_k, kps_un, sizeof(sgs_keypoint) * N); up(d_ur, uright, 4 * N); up(d_xyz, xyz, 12 * N); up(d_Tin, tcw_in, 64); up(d_n, &n, 4); up(d_has, has_mp, N);
-    if (e == cudaSuccess) e = cudaMemset(d_out, 0, N);
-    int rc = SGS_OK;
-    if (e == cudaSuccess) {
-        sgs_poseopt_batch b;
-        b.cam = *cam; b.tcw_in = d_Tin; b.kps = d_k; b.uright = d_ur; b.n = d_n; b.cap = n; b.has_mp = d_has; b.mp_index = nullptr; b.points_xyz = d_xyz; b.point_cap = n;
-        for (int l = 0; l < 16; ++l) b.inv_level_sigma2[l] = inv_level_sigma2[l];
-        b.tcw_out = d_Tout; b.outlier = d_out; b.ninliers = d_nin; b.scratch_err = d_err; b.scratch_level = d_lvl;
-        b.points2_xyz = nullptr; b.id_base2 = 0; b.point2_cap = 0;
-        rc = sgs_pose_optimization_batch_device(&b, 1, nullptr);
-        if (rc == SGS_OK) {
-            e = cudaMemcpy(tcw_out, d_Tout, 64, cudaMemcpyDeviceToHost);
-            if (e == cudaSuccess) e = cudaMemcpy(outlier, d_out, N, cudaMemcpyDeviceToHost);
-            int32_t nin = 0;
-            if (e == cudaSuccess) e = cudaMemcpy(&nin, d_nin, 4, cudaMemcpyDeviceToHost);
-            *ninliers = nin;
-        }
-    }
-    cudaFree(d);
-    if (rc != SGS_OK) return rc;
-    if (e != cudaSuccess) { set_error("sgs_pose_optimization: %s", cudaGetErrorString(e)); return SGS_ERR_CUDA; }
-    return SGS_OK;
+    HostCall c("sgs_pose_optimization");
+    sgs_poseopt_batch b;
+    c.in(&b.tcw_in, tcw_in, 16); c.in(&b.kps, kps_un, n); c.in(&b.uright, uright, n); c.in(&b.n, &n, 1); c.in(&b.has_mp, has_mp, n);
+    c.in(&b.points_xyz, xyz, 3 * (size_t)n);
+    c.out(&b.tcw_out, tcw_out, 16); c.out(&b.outlier, outlier, n, true); c.out(&b.ninliers, ninliers, 1);
+    c.out(&b.scratch_err, nullptr, 3 * (size_t)n); c.out(&b.scratch_level, nullptr, n);
+    b.cam = *cam; b.cap = n; b.mp_index = nullptr; b.point_cap = n;
+    for (int l = 0; l < 16; ++l) b.inv_level_sigma2[l] = inv_level_sigma2[l];
+    b.points2_xyz = nullptr; b.id_base2 = 0; b.point2_cap = 0;
+    if (int rc = c.upload()) return rc;
+    if (int rc = sgs_pose_optimization_batch_device(&b, 1, nullptr)) return rc;
+    return c.download();
 }
 
 }  // extern "C"

@@ -21,7 +21,7 @@ from pysgs import binding as B
 B.LIB_PATH = '/tmp/sgs_asan/libsgs_cuda.so'
 import pytest
 t = R + '/tests/'
-sys.exit(pytest.main(['-q', '-x', '-p', 'no:cacheprovider', t + 'test_fuzz_readers.py', t + 'test_vocabulary_files.py', t + 'test_settings.py', t + 'test_abi_symbols.py', t + 'test_detector.py',
+sys.exit(pytest.main(['-q', '-x', '-p', 'no:cacheprovider', t + 'test_fuzz_readers.py', t + 'test_vocabulary_files.py', t + 'test_settings.py', t + 'test_abi_symbols.py', t + 'test_host_wrappers.py', t + 'test_detector.py',
                       '-k', 'not batched_cpu and not product_never']))
 PY
 export LD_PRELOAD="$(gcc -print-file-name=libasan.so) $(gcc -print-file-name=libubsan.so)" ASAN_OPTIONS=detect_leaks=0 UBSAN_OPTIONS=print_stacktrace=1
